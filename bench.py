@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torchrun, one rank per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W
     python bench.py --config r50fpn2d | r18tube               (BASELINE.json configs[1] / configs[2])
+    python bench.py ... --dump-outputs DIR                    (the last timed step's detections as DIR/*.npy)
 
 Workload (config.workload), default = BASELINE.json configs[3]: 3-D ResNet-50-FPN (T=3, time kernel 3) keypoint
 R-CNN inference, 800x1333 frames (blob 800x1344), per-clip data parallel: FPN3D body, BODY_HEAD_LINK slice-center,
@@ -188,25 +189,16 @@ def run_reference(args):
     cores = pick_cpu_threads(torch)
     T = frames_per_clip(cfg)
     frames = synth_frames(1, T, args.height, args.width, 7)
-    steps, warm = max(args.steps, 1), max(args.warmup, 0)
-    # bounded sample: ONE clip per step; cap the run at ~5 minutes
-    t_first = None
-    done, t_total = 0, 0.0
-    for i in range(warm + steps):
-        t0 = time.time()
+    done = args.steps                       # ONE clip per step
+    for _ in range(args.warmup):
         reference_clip(cfg, blobs, frames)
-        dt = time.time() - t0
-        if t_first is None:
-            t_first = dt
-        if i >= warm:
-            done += 1; t_total += dt
-        if (i + 1 < warm + steps) and (time.time() - T_START + dt > 300):
-            break
-    if done == 0:
-        done, t_total = 1, t_first
+    t0 = time.time()
+    for _ in range(done):
+        reference_clip(cfg, blobs, frames)
+    t_total = time.time() - t0
     v = done / t_total
     line = dict(impl='reference', metric='clips/sec (T=3, 800x1333)', value=v, unit='clips/s', n_gpus=args.gpus,
-                steps=done, warmup=min(warm, 1), ms_per_step=1000.0 * t_total / done, higher_is_better=True, scaling='weak',
+                steps=done, warmup=args.warmup, ms_per_step=1000.0 * t_total / done, higher_is_better=True, scaling='weak',
                 vs_baseline=None, dtype='f32', data='synthetic',
                 config=dict(workload=WORKLOADS[args.config] % (args.height, args.width),
                             clips_per_step=1, note='torch-fp32 CPU restatement of the reference graph + reference host ops (oracle/); '
@@ -284,6 +276,30 @@ class ConvMeter(object):
         return rows
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, out, num_classes):
+    """What a caller of the captured step receives (engine.gather / ClipPipeline read the same rows), as .npy files:
+    det_counts [B, C-1], boxes [sum of counts, 5] and keypoints [sum of class-1 counts, 4, K], clip by clip, then class.
+    Beyond DUMP_BYTES, a fixed seeded subset of the clips is written; clip_index lists the clips kept."""
+    dets = out['dets'].float().cpu().numpy()                              # [B, C-1, cap, 5]
+    B, cap = dets.shape[0], dets.shape[2]
+    cnt = np.minimum(out['det_counts'].view(B, num_classes - 1).cpu().numpy(), cap)
+    xy = None if out['xy'] is None else out['xy'].float().cpu().numpy().reshape((B, cap) + tuple(out['xy'].shape[1:]))
+    per_clip = 8 * (num_classes - 1) + dets[0].nbytes + (0 if xy is None else xy[0].nbytes)
+    keep = np.arange(B)
+    if B * per_clip > DUMP_BYTES:
+        keep = np.sort(np.random.RandomState(0).choice(B, DUMP_BYTES // per_clip, replace=False))
+    arrays = dict(clip_index=keep.astype(np.float64), det_counts=cnt[keep].astype(np.float64),
+                  boxes=np.concatenate([dets[b, j, :cnt[b, j]] for b in keep for j in range(num_classes - 1)]))
+    if xy is not None:
+        arrays['keypoints'] = np.concatenate([xy[b, :cnt[b, 0]] for b in keep])
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + '.npy'), a)
+
+
 def measure_mode(mode, cfg, blobs, args, ctx, full):
     """One arithmetic mode: captured step (ClipPipeline), resident + API end-to-end timing; full: also the launch count,
     the eager roofline pass and (rank 0) clock sampling."""
@@ -327,10 +343,12 @@ def measure_mode(mode, cfg, blobs, args, ctx, full):
     e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step_resident()
+        out = step_resident()
     e1.record()
     barrier()
     res['ms'] = e0.elapsed_time(e1)
+    if full and args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, eng.spec.num_classes)
     # ---- end to end through the API: host numpy clips -> ClipPipeline.run -> the reference's per-clip containers ----
     got = []
 
@@ -458,7 +476,7 @@ def run_ours(args):
         try:
             import gc
             gc.collect(); torch.cuda.empty_cache()
-            tl = _train_measure(args, rank, world, local, steps=min(args.steps, 10))
+            tl = _train_measure(args, rank, world, local)
             if tl is not None:
                 training = dict(metric=tl['metric'], value=tl['value'], unit=tl['unit'], ms_per_step=tl['ms_per_step'], n_gpus=world,
                                 dtype='bf16', e2e=tl['e2e'], roofline=dict(achieved=tl['roofline']['achieved'], frac=tl['roofline']['frac'],
@@ -543,7 +561,7 @@ def synth_gt(B, H, W, seed, G=4, K=17):
     return entries
 
 
-def _train_measure(args, rank, world, local, steps=None):
+def _train_measure(args, rank, world, local):
     """One measured training leg on an initialised process group (all ranks call it); returns the JSON line as a dict on rank 0,
     None elsewhere.  `--train`: BASELINE.json configs[4], the keypoint R-CNN training step (modeling/trainer.KeypointRcnnTrainer): frozen
     stem, bf16 forward of res3..res5 + FPN3D + RPN + both RoI heads, ALL targets generated on the device (RPN anchor targets,
@@ -554,7 +572,7 @@ def _train_measure(args, rank, world, local, steps=None):
     import torch.distributed as dist
     from detectandtrack_b200.modeling import params as P
     from detectandtrack_b200.modeling.trainer import RpnTrainer, KeypointRcnnTrainer, pack_gt
-    nsteps = steps or args.steps
+    nsteps = args.steps
     cfg = bench_cfg(args.height, args.width, 'r50fpn3d')
     cfg.TRAIN.BATCH_SIZE_PER_IM = 512; cfg.TRAIN.RPN_PRE_NMS_TOP_N = 2000      # the shipped keypoint yamls (configs/video/2d_best)
     blobs, spec = P.random_blobs(cfg)
@@ -758,13 +776,11 @@ def tracking_leg(videos=64, frames=30, dets=100, cpu_videos=4):
         cfg.TRACKING.DISTANCE_METRICS, cfg.TRACKING.DISTANCE_METRIC_WTS, cfg.TRACKING.BIPARTITE_MATCHING_ALGO = saved
 
 
-T_START = time.time()
-
 if __name__ == '__main__':
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=10)
-    ap.add_argument('--warmup', type=int, default=3)
+    ap.add_argument('--steps', type=int, default=None, help='timed steps (default 10; --impl reference: 2)')
+    ap.add_argument('--warmup', type=int, default=None, help='warm-up steps (default 3; --impl reference: 1)')
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--dtype', default='auto', choices=['auto', 'bf16', 'tf32', 'tf32x3', 'bf16x3', 'bf16x3h'],
                     help='auto: headline bf16x3 (the parity mode) + bf16 / tf32 as labelled extras')
@@ -780,12 +796,21 @@ if __name__ == '__main__':
     ap.add_argument('--train', action='store_true', help='BASELINE.json configs[4]: keypoint R-CNN training step with NCCL gradient all-reduce (see run_train)')
     ap.add_argument('--train-trunk', action='store_true', help='with --train: the RPN-model trunk alone')
     ap.add_argument('--buckets', type=int, default=4, help='--train: gradient all-reduce buckets')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps, write the detections of the last step '
+                    '(det_counts, boxes, keypoints, clip_index) as DIR/<name>.npy')
     a = ap.parse_args()
+    reference = a.impl == 'reference' and not a.train
+    if a.steps is None:
+        a.steps = 2 if reference else 10
+    if a.warmup is None:
+        a.warmup = 1 if reference else 3
+    if a.steps < 1 or a.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    if a.dump_outputs and (a.train or reference):
+        ap.error('--dump-outputs applies to the inference benchmark (--impl ours, no --train)')
     if a.train:
         run_train(a)
-    elif a.impl == 'reference':
-        if a.steps == 10 and a.warmup == 3:
-            a.steps, a.warmup = 2, 1
+    elif reference:
         run_reference(a)
     else:
         run_ours(a)

@@ -1,20 +1,12 @@
 """CPU: the oracle restatements vs goldens produced by the reference's own code
-(tests/golden/gen_golden.py) and vs the compiled reference Cython (oracle/_ref)
-when it is present.  Integer outputs must be identical; fp32 outputs bit-equal
-unless a tolerance is stated."""
-import importlib
+(tests/golden/gen_golden.py) and by the compiled reference Cython
+(tests/golden/gen_golden_compiled.py).  Integer outputs must be identical; fp32
+outputs bit-equal unless a tolerance is stated."""
 import numpy as np
 import pytest
 
 from oracle import boxes as ob
 from oracle import proposals as op
-
-
-def _ref(name):
-    try:
-        return importlib.import_module('oracle._ref.' + name)
-    except Exception:
-        return None
 
 
 def test_iou_golden(golden):
@@ -26,15 +18,11 @@ def test_iou_golden(golden):
     assert np.array_equal(ob.bbox_overlaps(g['iou5_a'], g['iou5_b']), g['iou5_out'])
 
 
-def test_iou_vs_compiled_reference():
-    cb = _ref('cython_bbox')
-    if cb is None:
-        pytest.skip('oracle/_ref not built (reference absent)')
-    rng = np.random.default_rng(5)
-    for scale in (0.02, 1.0, 7.0):
-        x1 = rng.uniform(0, 500, 400); y1 = rng.uniform(0, 300, 400)
-        a = np.stack([x1, y1, x1 + rng.uniform(0, 200, 400) * scale, y1 + rng.uniform(0, 200, 400) * scale], 1).astype(np.float32)
-        assert np.array_equal(cb.bbox_overlaps(a[:250], a[250:]), ob.bbox_overlaps_2d(a[:250], a[250:]))
+def test_iou_vs_compiled_reference(golden):
+    g = golden('compiled_ref')
+    for i in range(3):                                  # box size scales 0.02, 1, 7
+        a = g['iou%d_boxes' % i]
+        assert np.array_equal(g['iou%d_out' % i], ob.bbox_overlaps_2d(a[:250], a[250:]))
 
 
 def test_iou_edge_cases():
@@ -54,17 +42,11 @@ def test_nms_golden(golden, name):
         assert np.array_equal(keep, g['%s_keep_%d' % (name, int(th * 10))])
 
 
-def test_nms_vs_compiled_reference():
-    cn = _ref('cython_nms')
-    if cn is None:
-        pytest.skip('oracle/_ref not built (reference absent)')
-    rng = np.random.default_rng(7)
-    c = rng.uniform(0, 600, (60, 2))
-    xy = c[rng.integers(0, 60, 1500)] + rng.normal(0, 12, (1500, 2))
-    wh = rng.uniform(20, 120, (1500, 2))
-    d = np.hstack([xy, xy + wh, rng.permutation(1500)[:, None] / 1500.]).astype(np.float32)
+def test_nms_vs_compiled_reference(golden):
+    g = golden('compiled_ref')
+    d = g['nms_dets']
     for th in (0.3, 0.7):
-        assert np.array_equal(cn.nms(d, np.float32(th)), ob.nms_2d(d, th))
+        assert np.array_equal(g['nms_keep_%d' % int(th * 10)], ob.nms_2d(d, th))
 
 
 def test_nms_empty_and_single():
