@@ -1,4 +1,4 @@
-"""ctypes binding of libdt_b200.so (include/dt_b200.h).  No torch types cross
+"""ctypes binding of libdt_b200.so (include/dt_b200.h, include/dt_b200_train3d.h).  No torch types cross
 the boundary: tensors are passed as raw device pointers + sizes + stream."""
 import ctypes as C
 import os
@@ -68,6 +68,12 @@ SIGNATURES = {
     'dt_sample_rois': [_p, _p, _p, _i, _i, _i, _p, _p, _p, _p, _p, _i, _i, _i, _p, _i, _i, _f, _f, _f, _f, C.POINTER(_f), _i,
                        C.c_ulonglong, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i, _p, _p],
 }
+# the tube model's training-step entry points (include/dt_b200_train3d.h), error-code functions like the above
+TRAIN3D_SIGNATURES = {
+    'dt_rpn_tube_loss_grad': [_p, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _f, _f, _f, _p, _p, _i, _p, _p],
+    'dt_frcnn_tube_loss_grad': [_p, _i, _p, _p, _p, _p, _i, _i, _i, _p, _f, _f, _p, _i, _p, _p, _p],
+    'dt_spatial_mean_bwd': [_p, C.c_longlong, _i, _i, _i, _p, _p, _p, _p, _p, _p],
+}
 # host-only helpers (not error-code functions)
 HOST_FUNCS = {'dt_planes_ld': ([_i, _i, _i, _i], C.c_int), 'dt_jpeg_available': ([], C.c_int)}
 
@@ -121,7 +127,7 @@ def lib():
         l = C.CDLL(LIB_PATH)
         l.dt_last_error.restype = C.c_char_p
         l.dt_last_error.argtypes = []
-        for name, args in SIGNATURES.items():
+        for name, args in list(SIGNATURES.items()) + list(TRAIN3D_SIGNATURES.items()):
             fn = getattr(l, name)
             fn.argtypes = args
             fn.restype = _RESTYPE.get(name, C.c_int)

@@ -34,7 +34,7 @@ def build_lib(force=False, verbose=False):
     os.makedirs(OBJ, exist_ok=True)
     os.makedirs(LIBDIR, exist_ok=True)
     headers = tuple(os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith(('.cuh', '.h')))
-    headers += (os.path.join(ROOT, 'include', 'dt_b200.h'),)
+    headers += tuple(os.path.join(ROOT, 'include', f) for f in os.listdir(os.path.join(ROOT, 'include')) if f.endswith('.h'))
     srcs = sorted(f for f in os.listdir(CSRC) if f.endswith('.cu'))
     jobs = []
     objs = []

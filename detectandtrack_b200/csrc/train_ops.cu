@@ -25,6 +25,7 @@
 #include "common.cuh"
 #include "tc_common.cuh"
 #include "../../include/dt_b200.h"
+#include "../../include/dt_b200_train3d.h"
 #include <cuda_bf16.h>
 #include <stdlib.h>
 
@@ -670,6 +671,107 @@ __global__ void rpn_loss_grad_kernel(const float* __restrict__ out, int ld_o, co
   if ((threadIdx.x & 31) == 0 && loss) { if (lc != 0.f) atomicAdd(loss, lc); if (lb != 0.f) atomicAdd(loss + 1, lb); }
 }
 
+// The normaliser of Detectron's SigmoidCrossEntropyLoss with its default normalize=1: max(#labels >= 0, 1e-5) over the
+// whole label blob.  One CTA (the single-level tube RPN has a few 10^4 labels per GPU).
+__global__ void __launch_bounds__(1024) label_count_kernel(const int* __restrict__ labels, long long n, float* __restrict__ norm) {
+  __shared__ int part[32];
+  int c = 0;
+  for (long long i = threadIdx.x; i < n; i += blockDim.x) c += labels[i] >= 0;
+  for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
+  if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = c;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    int s = 0;
+    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s += part[w];
+    norm[0] = fmaxf((float)s, 1e-5f);
+  }
+}
+
+// Tube RPN losses (model_builder.py add_rpn_outputs(nd=True) + add_rpn_losses(time_dim=T)) read from the per-frame head
+// output out [B, T, HW, ld_o] fp32 = [A logits | 4A deltas (a*4 + k)] per frame:
+//   cls   TimePool avg of the logits over T, SigmoidCrossEntropyLoss(scale = s_cls) / norm[0]   labels [B, HW, A]
+//   bbox  SmoothL1Loss(beta, scale = s_box) on the frame-folded deltas: channel a*4 + k of frame t is column
+//         a*4T + t*4 + k of targets / inside / outside [B, HW, 4TA]
+// grad [B, T, HW, ld_g] bf16 in the per-frame layout: the TimePool backward puts the logit gradient / T on every frame.
+__global__ void rpn_tube_loss_grad_kernel(const float* __restrict__ out, int ld_o, const int* __restrict__ labels,
+                                          const float* __restrict__ targets, const float* __restrict__ iw, const float* __restrict__ ow,
+                                          int B, int T, long long HW, int A, float s_cls, float s_box, float beta,
+                                          const float* __restrict__ norm, __nv_bfloat16* __restrict__ grad, int ld_g, float* __restrict__ loss) {
+  float lc = 0.f, lb = 0.f;
+  const long long total = (long long)B * T * HW * ld_g;
+  const float sc = s_cls / norm[0];
+  for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
+    const int ch = (int)(idx % ld_g);
+    const long long q = idx / ld_g;
+    const long long p = q % HW;
+    const int t = (int)((q / HW) % T), b = (int)(q / HW / T);
+    const long long pix = (long long)b * HW + p;
+    float gv = 0.f;
+    if (ch < A) {
+      const int lab = labels[pix * A + ch];
+      if (lab >= 0) {
+        const float* o = out + ((size_t)b * T * HW + p) * ld_o + ch;
+        float x = o[0];
+        for (int u = 1; u < T; ++u) x += o[(size_t)u * HW * ld_o];
+        x /= (float)T;
+        if (t == 0) lc += sc * (-x * ((float)lab - (x >= 0.f ? 1.f : 0.f)) + log1pf(expf(x - 2.f * x * (x >= 0.f ? 1.f : 0.f))));
+        gv = sc * (1.f / (1.f + expf(-x)) - (float)lab) / (float)T;
+      }
+    } else if (ch < 5 * A) {
+      const int j = ch - A;
+      const size_t col = (size_t)pix * 4 * T * A + (j >> 2) * 4 * T + t * 4 + (j & 3);
+      const float w_in = iw[col], w_out = ow[col];
+      const float d = w_in * (out[(size_t)q * ld_o + ch] - targets[col]);
+      const float ad = fabsf(d);
+      lb += s_box * w_out * (ad < beta ? 0.5f * d * d / beta : ad - 0.5f * beta);
+      gv = s_box * w_out * w_in * (ad < beta ? d / beta : (d > 0.f ? 1.f : -1.f));
+    }
+    grad[idx] = __float2bfloat16_rn(gv);
+  }
+  for (int o = 16; o > 0; o >>= 1) { lc += __shfl_xor_sync(0xffffffffu, lc, o); lb += __shfl_xor_sync(0xffffffffu, lb, o); }
+  if ((threadIdx.x & 31) == 0 && loss) { if (lc != 0.f) atomicAdd(loss, lc); if (lb != 0.f) atomicAdd(loss + 1, lb); }
+}
+
+// Backward of the two ReduceBackMeans (W, then H) of the res5 RoI head, fused with the pointwise step that follows it:
+// out[n, p, c] = g[n, c] / HW * [y > 0] * scale[c]; out2 = the same masked value * scale2[c] (or unscaled).  y, scale, out2
+// may be NULL (plain broadcast).  The [N, HW, C] broadcast itself is never stored.
+__global__ void spatial_mean_bwd_kernel(const __nv_bfloat16* __restrict__ g, long long N, int HW, int C, const __nv_bfloat16* __restrict__ y,
+                                        const float* __restrict__ scale, __nv_bfloat16* __restrict__ out, const float* __restrict__ scale2,
+                                        __nv_bfloat16* __restrict__ out2) {
+  const int cv = C / 8;
+  const long long total = N * HW * cv;
+  const float inv = 1.f / (float)HW;
+  for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
+    const int c = (int)(idx % cv) * 8;
+    const long long row = idx / cv;
+    const size_t off = (size_t)row * C + c;
+    const uint4 a = *reinterpret_cast<const uint4*>(g + (size_t)(row / HW) * C + c);
+    const __nv_bfloat16* ae = reinterpret_cast<const __nv_bfloat16*>(&a);
+    float v[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) v[j] = __bfloat162float(ae[j]) * inv;
+    if (y) {
+      const uint4 m = *reinterpret_cast<const uint4*>(y + off);
+      const __nv_bfloat16* me = reinterpret_cast<const __nv_bfloat16*>(&m);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) v[j] = __bfloat162float(me[j]) > 0.f ? v[j] : 0.f;
+    }
+    __align__(16) __nv_bfloat16 o[8];
+    if (out2) {
+#pragma unroll
+      for (int j = 0; j < 8; ++j) o[j] = __float2bfloat16_rn(scale2 ? v[j] * scale2[c + j] : v[j]);
+      *reinterpret_cast<uint4*>(out2 + off) = *reinterpret_cast<const uint4*>(o);
+    }
+    if (scale) {
+#pragma unroll
+      for (int j = 0; j < 8; ++j) v[j] *= scale[c + j];
+    }
+#pragma unroll
+    for (int j = 0; j < 8; ++j) o[j] = __float2bfloat16_rn(v[j]);
+    *reinterpret_cast<uint4*>(out + off) = *reinterpret_cast<const uint4*>(o);
+  }
+}
+
 
 // ------------------------------------------------------------------------------------------------ RoI heads (backward)
 // out = bf16(g + acc)
@@ -760,40 +862,57 @@ __global__ void roi_align_bwd_kernel(RoiBwdLevels lv, int kmin, const float* __r
   }
 }
 
-// one thread per RoI row (C is small)
+// one thread per RoI (C is small).  A RoI owns T consecutive rows of `out` / `grad`, one per frame, each [C logits |
+// 4C deltas (c*4 + k)]; T = 1 is the 2-D head.  For T > 1 the fold of dt_fold_tube_heads is applied on the fly (logits =
+// mean over the frames, box column c*4T + t*4 + k of targets / weights) and its backward is fused into the gradient
+// write: every frame row receives the logit gradient / T and its own frame's box gradient.  With T = 1 every
+// expression reduces exactly (x / 1.f == x) to the 2-D head's.
+__device__ __forceinline__ float tube_logit(const float* o, int ld_o, int T, int j) {
+  float a = o[j];
+  for (int t = 1; t < T; ++t) a += o[(size_t)t * ld_o + j];
+  return a / (float)T;
+}
+
 __global__ void frcnn_loss_grad_kernel(const float* __restrict__ out, int ld_o, const int* __restrict__ labels,
                                        const float* __restrict__ targets, const float* __restrict__ iw, const float* __restrict__ ow,
-                                       int rows, int C, const float* __restrict__ totals, float s_cls, float s_box,
+                                       int rows, int T, int C, const float* __restrict__ totals, float s_cls, float s_box,
                                        __nv_bfloat16* __restrict__ grad, int ld_g, float* __restrict__ loss, float* __restrict__ acc) {
   const int r = blockIdx.x * blockDim.x + threadIdx.x;
   float lc = 0.f, lb = 0.f, hit = 0.f;
   if (r < rows) {
-    __nv_bfloat16* g = grad + (size_t)r * ld_g;
+    __nv_bfloat16* g = grad + (size_t)r * T * ld_g;
     const int lbl = labels[r];
     const float N = totals[0];
     if (lbl < 0 || !(N > 0.f)) {
-      for (int j = 0; j < ld_g; ++j) g[j] = __float2bfloat16_rn(0.f);
+      for (int j = 0; j < T * ld_g; ++j) g[j] = __float2bfloat16_rn(0.f);
     } else {
-      const float* o = out + (size_t)r * ld_o;
-      float m = o[0]; int am = 0;
-      for (int j = 1; j < C; ++j) if (o[j] > m) { m = o[j]; am = j; }
+      const float* o = out + (size_t)r * T * ld_o;
+      const int C4T = 4 * C * T;
+      float m = tube_logit(o, ld_o, T, 0); int am = 0;
+      for (int j = 1; j < C; ++j) { const float v = tube_logit(o, ld_o, T, j); if (v > m) { m = v; am = j; } }
       float se = 0.f;
-      for (int j = 0; j < C; ++j) se += expf(o[j] - m);
+      for (int j = 0; j < C; ++j) se += expf(tube_logit(o, ld_o, T, j) - m);
       const float lse = logf(se);
-      lc = -(o[lbl] - m - lse) * s_cls / N;
+      lc = -(tube_logit(o, ld_o, T, lbl) - m - lse) * s_cls / N;
       hit = am == lbl ? 1.f : 0.f;
       for (int j = 0; j < C; ++j) {
-        const float pj = expf(o[j] - m - lse);
-        g[j] = __float2bfloat16_rn((pj - (j == lbl ? 1.f : 0.f)) * s_cls / N);
+        const float pj = expf(tube_logit(o, ld_o, T, j) - m - lse);
+        const __nv_bfloat16 gj = __float2bfloat16_rn((pj - (j == lbl ? 1.f : 0.f)) * s_cls / N / (float)T);
+        for (int t = 0; t < T; ++t) g[(size_t)t * ld_g + j] = gj;
       }
-      for (int j = 0; j < 4 * C; ++j) {
-        const float w_in = iw[(size_t)r * 4 * C + j], w_out = ow[(size_t)r * 4 * C + j];
-        const float d = w_in * (o[C + j] - targets[(size_t)r * 4 * C + j]);
-        const float ad = fabsf(d);
-        lb += w_out * (ad < 1.f ? 0.5f * d * d : ad - 0.5f) * s_box / N;
-        g[C + j] = __float2bfloat16_rn(w_out * w_in * (ad < 1.f ? d : (d > 0.f ? 1.f : -1.f)) * s_box / N);
+      for (int t = 0; t < T; ++t) {
+        const float* ot = o + (size_t)t * ld_o;
+        __nv_bfloat16* gt = g + (size_t)t * ld_g;
+        for (int j = 0; j < 4 * C; ++j) {
+          const size_t col = (size_t)r * C4T + (j >> 2) * 4 * T + t * 4 + (j & 3);
+          const float w_in = iw[col], w_out = ow[col];
+          const float d = w_in * (ot[C + j] - targets[col]);
+          const float ad = fabsf(d);
+          lb += w_out * (ad < 1.f ? 0.5f * d * d : ad - 0.5f) * s_box / N;
+          gt[C + j] = __float2bfloat16_rn(w_out * w_in * (ad < 1.f ? d : (d > 0.f ? 1.f : -1.f)) * s_box / N);
+        }
+        for (int j = 5 * C; j < ld_g; ++j) gt[j] = __float2bfloat16_rn(0.f);
       }
-      for (int j = 5 * C; j < ld_g; ++j) g[j] = __float2bfloat16_rn(0.f);
     }
   }
   for (int o2 = 16; o2 > 0; o2 >>= 1) {
@@ -1174,8 +1293,48 @@ extern "C" int dt_frcnn_loss_grad(const float* out, int ld_o, const int* labels,
   DT_CHECK_ARG(rows >= 0 && C >= 2 && ld_o >= 5 * C && ld_g >= 5 * C, "dt_frcnn_loss_grad: bad shape rows=%d C=%d ld_o=%d ld_g=%d", rows, C, ld_o, ld_g);
   if (rows == 0) return 0;
   DT_CHECK_ARG(out && labels && targets && inside_w && outside_w && totals && grad, "dt_frcnn_loss_grad: null pointer");
-  frcnn_loss_grad_kernel<<<(rows + 127) / 128, 128, 0, (cudaStream_t)stream>>>(out, ld_o, labels, targets, inside_w, outside_w, rows, C, totals,
-                                                                             scale_cls, scale_box, (__nv_bfloat16*)grad, ld_g, loss, accuracy);
+  frcnn_loss_grad_kernel<<<(rows + 127) / 128, 128, 0, (cudaStream_t)stream>>>(out, ld_o, labels, targets, inside_w, outside_w, rows, 1, C,
+                                                                             totals, scale_cls, scale_box, (__nv_bfloat16*)grad, ld_g, loss, accuracy);
+  DT_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int dt_frcnn_tube_loss_grad(const float* out, int ld_o, const int* labels, const float* targets, const float* inside_w,
+                                       const float* outside_w, int R, int T, int C, const float* totals, float scale_cls, float scale_box,
+                                       void* grad, int ld_g, float* loss, float* accuracy, void* stream) {
+  DT_CHECK_ARG(R >= 0 && T >= 1 && T <= DT_MAX_T && C >= 2 && ld_o >= 5 * C && ld_g >= 5 * C,
+               "dt_frcnn_tube_loss_grad: bad shape R=%d T=%d C=%d ld_o=%d ld_g=%d", R, T, C, ld_o, ld_g);
+  if (R == 0) return 0;
+  DT_CHECK_ARG(out && labels && targets && inside_w && outside_w && totals && grad, "dt_frcnn_tube_loss_grad: null pointer");
+  frcnn_loss_grad_kernel<<<(R + 127) / 128, 128, 0, (cudaStream_t)stream>>>(out, ld_o, labels, targets, inside_w, outside_w, R, T, C,
+                                                                          totals, scale_cls, scale_box, (__nv_bfloat16*)grad, ld_g, loss, accuracy);
+  DT_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int dt_rpn_tube_loss_grad(const float* out, int ld_o, const int* labels, const float* targets, const float* inside_w,
+                                     const float* outside_w, int B, int T, int H, int W, int A, float scale_cls, float scale_box, float beta,
+                                     float* normalizer, void* grad, int ld_g, float* loss, void* stream) {
+  DT_CHECK_ARG(B >= 0 && T >= 1 && T <= DT_MAX_T && H >= 1 && W >= 1 && A >= 1 && ld_o >= 5 * A && ld_g >= 5 * A && beta > 0.f,
+               "dt_rpn_tube_loss_grad: bad shape B=%d T=%d %dx%d A=%d ld_o=%d ld_g=%d", B, T, H, W, A, ld_o, ld_g);
+  if (B == 0) return 0;
+  DT_CHECK_ARG(out && labels && targets && inside_w && outside_w && normalizer && grad, "dt_rpn_tube_loss_grad: null pointer");
+  const long long HW = (long long)H * W;
+  label_count_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(labels, (long long)B * HW * A, normalizer);
+  DT_CHECK_LAUNCH();
+  rpn_tube_loss_grad_kernel<<<grid_for((long long)B * T * HW * ld_g, 256), 256, 0, (cudaStream_t)stream>>>(
+      out, ld_o, labels, targets, inside_w, outside_w, B, T, HW, A, scale_cls, scale_box, beta, normalizer, (__nv_bfloat16*)grad, ld_g, loss);
+  DT_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int dt_spatial_mean_bwd(const void* g, long long N, int H, int W, int C, const void* y, const float* scale, void* out,
+                                   const float* scale2, void* out2, void* stream) {
+  DT_CHECK_ARG(N >= 0 && H >= 1 && W >= 1 && C >= 8 && C % 8 == 0, "dt_spatial_mean_bwd: bad shape N=%lld %dx%d C=%d (C %% 8 == 0)", N, H, W, C);
+  if (N == 0) return 0;
+  DT_CHECK_ARG(g && out, "dt_spatial_mean_bwd: null pointer");
+  spatial_mean_bwd_kernel<<<grid_for(N * H * W * (C / 8), 256), 256, 0, (cudaStream_t)stream>>>(
+      (const __nv_bfloat16*)g, N, H * W, C, (const __nv_bfloat16*)y, scale, (__nv_bfloat16*)out, scale2, (__nv_bfloat16*)out2);
   DT_CHECK_LAUNCH();
   return 0;
 }

@@ -57,6 +57,9 @@ def create(model_name, train=False, init_params=None, blobs=None, dtype=None):
         if model_name == 'rpn':
             return T.RpnTrainer(cfg, blobs, spec, world=world)
         if model_name == 'keypoint_rcnn' and cfg.MODEL.FASTER_RCNN and cfg.MODEL.KEYPOINTS_ON:
+            if spec.head3d:                                   # single-level 3-D body with tube heads
+                from .tube_trainer import TubeKeypointRcnnTrainer
+                return TubeKeypointRcnnTrainer(cfg, blobs, spec, world=world)
             return T.KeypointRcnnTrainer(cfg, blobs, spec, world=world)
         raise NotImplementedError('training graph for MODEL.TYPE {!r}'.format(model_name))
     if model_name not in _GENERIC_TYPES:

@@ -21,7 +21,9 @@ and all on the device,
     kps head   RoIAlign 14x14 -> 8 x conv3x3 -> sub-pixel deconv, spatial SoftmaxWithLoss through the fixed bilinear 2x
                upsampling (dt_kps_loss_grad)
     backward   the FC / conv layers through the same dgrad / wgrad kernels (an FC is a 1x1 conv over the RoI axis),
-               dt_roi_align_bwd into fp32 per-level accumulators that join the RPN's feature gradients."""
+               dt_roi_align_bwd into fp32 per-level accumulators that join the RPN's feature gradients.
+
+The single-level 3-D bodies with tube heads (the R18-3D yaml) train through tube_trainer.TubeKeypointRcnnTrainer."""
 import os
 
 import numpy as np
@@ -124,21 +126,27 @@ class TrainConv(object):
     def backward(self, gz, x, x_planes=None, need_dx=True):
         """gz: gradient wrt the conv's raw output (after the pointwise joins), x: the saved input.  Accumulates dW (and db),
         returns (dx or None, x_planes)."""
-        N, T, Ho, Wo, _ = gz.shape
         assert self.cout % 8 == 0 and gz.shape[-1] == self.cout
+        stride = self.stride[1:]
+        spatial = self.stride[1] == 2 and self.k[1] > 1
+        if spatial:           # strided 3x3(x3) conv: with gz on the even positions of the input grid (zeros elsewhere) both
+            # gradients are stride-1 'same' ones: dx = conv(gz', flip(W)^T), dW[k] = sum_i gz'[i] x[i + k - pad]
+            gz = to.scatter_stride2(gz, (x.shape[2], x.shape[3]))
+            stride = (1, 1)
+        N, T, Ho, Wo, _ = gz.shape
         if WGRAD_PLANES:      # the first implementation: channel-major plane copies of both operands (kept for A/B runs)
             sp = (self.pad[1], self.pad[2])
             if x_planes is None:
-                x_planes = to.to_planes(x, pad=sp, stride=self.stride[1:], channels=self.cin, copies=True)
+                x_planes = to.to_planes(x, pad=sp, stride=stride, channels=self.cin, copies=True)
             to.wgrad(to.to_planes(gz, pad=sp), x_planes, (Ho, Wo), self.k, self.g)
         else:                 # operands read straight from NDHWC (MN-major tcgen05 operands, tap = TMA coordinate shift)
-            to.wgrad_nhwc(gz, x, self.k, self.stride[1:], self.g, cout=self.cout, cin=self.cin)
+            to.wgrad_nhwc(gz, x, self.k, stride, self.g, cout=self.cout, cin=self.cin)
         if self.bias is not None:
             L.call('dt_bias_grad', L.ptr(gz), gz.numel() // gz.shape[-1], self.cout, gz.shape[-1], L.ptr(self.bias_g), L.stream_ptr())
         dx = None
         if need_dx:
             dx = cv.conv3d(gz, self.w_dg, self.k, (1, 1, 1), self.pad, out_f32=False, dtype=cv.BF16, cin=self.cout)
-            if self.stride[1] == 2:
+            if self.stride[1] == 2 and not spatial:
                 dx = to.scatter_stride2(dx, (x.shape[2], x.shape[3]))
         return dx, x_planes
 
@@ -147,6 +155,44 @@ class TrainConv(object):
         if self.bias is not None:     # biases: no weight decay, 2x learning rate (model_builder.py:971-976)
             to.sgd_update(self.bias.view(1, 1, -1), self.bias_g.view(1, 1, -1), self.bias_m.view(1, 1, -1), 2.0 * lr, momentum, 0.0,
                           grad_scale)
+
+
+def _subpixel_taps():
+    """(sub-pixel filter (py, px), footprint tap (dy, dx), ConvTranspose tap (ky, kx)) of the k4-s2-p1 ConvTranspose written as
+    four 2x2 sub-pixel filters on one 3x3 footprint (engine.py)."""
+    for py in range(2):
+        for px in range(2):
+            for dy in (-1, 0, 1):
+                for dx in (-1, 0, 1):
+                    ky, kx = py + 1 - 2 * dy, px + 1 - 2 * dx
+                    if 0 <= ky <= 3 and 0 <= kx <= 3:
+                        yield py * 2 + px, dy + 1, dx + 1, ky, kx
+
+
+def subpixel_deconv_conv(torch, blobs):
+    """kps_score_lowres (ConvTranspose (Cin, K, 4, 4), stride 2, pad 1) as a trainable 3x3 conv with 4K (padded) outputs
+    -> (TrainConv, K, padded output count)."""
+    wt = blobs['kps_score_lowres_w']
+    cin, K = wt.shape[0], wt.shape[1]
+    ldk = (4 * K + 7) // 8 * 8
+    w3 = np.zeros((ldk, cin, 3, 3), np.float32)
+    for sub, ty, tx, ky, kx in _subpixel_taps():
+        w3[sub * K:(sub + 1) * K, :, ty, tx] = wt[:, :, ky, kx].T
+    b3 = np.zeros((ldk,), np.float32); b3[:4 * K] = np.tile(blobs['kps_score_lowres_b'], 4)
+    c = TrainConv(torch, w3, bias=b3)
+    c.cout_live = 4 * K
+    return c, K, ldk
+
+
+def export_subpixel_deconv(tr, blobs, out):
+    """The inverse of subpixel_deconv_conv on the trained master filter: kps_score_lowres_{w,b} into `out`."""
+    K = tr.K
+    w3 = tr._blob_w(tr.kps_lowres, (tr.kp_ld, tr.kps_lowres.cin, 3, 3))                 # [ldk, cin, 3, 3]
+    wt = np.zeros_like(blobs['kps_score_lowres_w'])                                      # (cin, K, 4, 4)
+    for sub, ty, tx, ky, kx in _subpixel_taps():
+        wt[:, :, ky, kx] = w3[sub * K:(sub + 1) * K, :, ty, tx].T
+    out['kps_score_lowres_w'] = wt
+    out['kps_score_lowres_b'] = tr.kps_lowres.bias.cpu().numpy()[:K].copy()
 
 
 class RpnTrainer(object):
@@ -196,7 +242,12 @@ class RpnTrainer(object):
         self.rpn_out._accumulate = self.rpn_conv._accumulate = 1
         self.convs.append(self.rpn_out)
         self._build_heads(blobs)                          # RoI heads of the full model (KeypointRcnnTrainer); none here
-        # ---- flat gradient buffer in BACKWARD order (so a bucket finished early in the backward pass is contiguous)
+        self._alloc_grads(buckets)
+
+    def _alloc_grads(self, buckets):
+        """The flat gradient buffer in BACKWARD order (so a bucket finished early in the backward pass is contiguous), its
+        all-reduce buckets and the loss accumulator."""
+        torch, world = self.torch, self.world
         order = self.convs[::-1]
         total = sum(c.nparams() for c in order)
         self.flat_g = torch.zeros(total, dtype=torch.float32, device='cuda')
@@ -391,9 +442,8 @@ class RpnTrainer(object):
         w = c.w.view(kT, kH, kW, c.cout, c.cin).permute(3, 4, 0, 1, 2).contiguous().cpu().numpy()
         return w.reshape((c.cout, c.cin) + tuple(shape[2:])) if len(shape) >= 2 else w
 
-    def export_blobs(self, blobs):
-        """The trained parameters written back into a copy of the weights dict under the reference's blob names
-        (lib/utils/net.py:252-294 save_model_to_weights_file): what tools/test_net.py loads through TEST.WEIGHTS."""
+    def _export_named(self, blobs):
+        """A copy of the weights dict with every conv that carries its blob name (filter and bias) replaced by its trained value."""
         out = dict(blobs)
         for c in self.convs:
             n = getattr(c, 'name', None)
@@ -402,6 +452,12 @@ class RpnTrainer(object):
             out[n + '_w'] = self._blob_w(c, blobs[n + '_w'].shape).astype(np.float32)
             if c.bias is not None:
                 out[n + '_b'] = c.bias.cpu().numpy()
+        return out
+
+    def export_blobs(self, blobs):
+        """The trained parameters written back into a copy of the weights dict under the reference's blob names
+        (lib/utils/net.py:252-294 save_model_to_weights_file): what tools/test_net.py loads through TEST.WEIGHTS."""
+        out = self._export_named(blobs)
         k = str(self.spec.rpn_levels[0])
         A = self.A
         w = self.rpn_out.w[0].cpu().numpy()                                   # [ld, Cin]
@@ -478,21 +534,27 @@ class RpnTrainer(object):
         return out
 
 
-def pack_gt(entries, Gmax=None, K=17):
+def pack_gt(entries, Gmax=None, K=17, device='cuda'):
     """roidb-style entries (dicts with 'boxes' [G,4] in ORIGINAL image coordinates, optional 'gt_classes', 'is_crowd',
     'gt_keypoints' [G,3,K] int32) -> the fixed-capacity device tensors of dt_rpn_targets / dt_sample_rois.  The RPN sees the
-    non-crowd boxes only (rpn.py:84-86), the RoI sampler all of them (json_dataset.py:437)."""
+    non-crowd boxes only (rpn.py:84-86), the RoI sampler all of them (json_dataset.py:437).
+    Tube entries (T > 1 frames): 'boxes' [G,4T] (frame t in columns 4t..4t+3), 'gt_keypoints' [G,3,K*T] (column t*K + k)
+    and an optional per-frame visibility 'gt_visible' [G,T]; the latter is returned as 'gt_visible' [B,Gmax,T] uint8,
+    aligned with 'rpn_boxes' (the boxes dt_rpn_targets reads)."""
     import torch
     B = len(entries)
     Gmax = Gmax or max(8, max(len(e['boxes']) for e in entries))
-    boxes = np.zeros((B, Gmax, 4), np.float32); rboxes = np.zeros((B, Gmax, 4), np.float32)
+    D = max(np.asarray(e['boxes']).reshape(len(e['boxes']), -1).shape[1] if len(e['boxes']) else 4 for e in entries)
+    T = D // 4
+    boxes = np.zeros((B, Gmax, D), np.float32); rboxes = np.zeros((B, Gmax, D), np.float32)
     classes = np.zeros((B, Gmax), np.int32); crowd = np.zeros((B, Gmax), np.int32)
-    kps = np.zeros((B, Gmax, 3, K), np.int32)
+    kps = np.zeros((B, Gmax, 3, K * T), np.int32)
+    vis = np.ones((B, Gmax, T), np.uint8)
     counts = np.zeros((B,), np.int32); rcounts = np.zeros((B,), np.int32)
     for b, e in enumerate(entries):
         g = len(e['boxes'])
         assert g <= Gmax, 'more gt boxes than Gmax'
-        boxes[b, :g] = e['boxes']
+        boxes[b, :g] = np.asarray(e['boxes'], np.float32).reshape(g, D)
         classes[b, :g] = e.get('gt_classes', np.ones(g, np.int32))
         cr = np.asarray(e.get('is_crowd', np.zeros(g, bool))).astype(bool)
         crowd[b, :g] = cr
@@ -502,9 +564,14 @@ def pack_gt(entries, Gmax=None, K=17):
         keep = np.where((classes[b, :g] > 0) & ~cr)[0]
         rboxes[b, :len(keep)] = boxes[b, keep]
         rcounts[b] = len(keep)
-    t = lambda a: torch.from_numpy(a).cuda()
-    return dict(boxes=t(boxes), classes=t(classes), crowd=t(crowd), keypoints=t(kps), counts=t(counts), rpn_boxes=t(rboxes),
-                rpn_counts=t(rcounts))
+        if 'gt_visible' in e:
+            vis[b, :len(keep)] = np.asarray(e['gt_visible']).reshape(g, T)[keep]
+    t = lambda a: torch.from_numpy(a).to(device)
+    out = dict(boxes=t(boxes), classes=t(classes), crowd=t(crowd), keypoints=t(kps), counts=t(counts), rpn_boxes=t(rboxes),
+               rpn_counts=t(rcounts))
+    if any('gt_visible' in e for e in entries):
+        out['gt_visible'] = t(vis)
+    return out
 
 
 class KeypointRcnnTrainer(RpnTrainer):
@@ -530,24 +597,7 @@ class KeypointRcnnTrainer(RpnTrainer):
         for i in range(cfg.KRCNN.NUM_STACKED_CONVS):
             c = TrainConv(torch, blobs['conv_fcn%d_w' % (i + 1)], bias=blobs['conv_fcn%d_b' % (i + 1)], relu=True)
             self.kps.append(c); add(c)
-        wt = blobs['kps_score_lowres_w']                      # ConvTranspose (Cin, K, 4, 4), stride 2, pad 1
-        cin, K = wt.shape[0], wt.shape[1]
-        self.K = K
-        ldk = self.kp_ld = (4 * K + 7) // 8 * 8
-        w3 = np.zeros((ldk, cin, 3, 3), np.float32)           # four 2x2 sub-pixel filters on one 3x3 footprint (engine.py)
-        for py in range(2):
-            for px in range(2):
-                for dy in (-1, 0, 1):
-                    ky = py + 1 - 2 * dy
-                    if not 0 <= ky <= 3:
-                        continue
-                    for dx in (-1, 0, 1):
-                        kx = px + 1 - 2 * dx
-                        if 0 <= kx <= 3:
-                            w3[(py * 2 + px) * K:(py * 2 + px + 1) * K, :, dy + 1, dx + 1] = wt[:, :, ky, kx].T
-        b3 = np.zeros((ldk,), np.float32); b3[:4 * K] = np.tile(blobs['kps_score_lowres_b'], 4)
-        self.kps_lowres = TrainConv(torch, w3, bias=b3); add(self.kps_lowres)
-        self.kps_lowres.cout_live = 4 * K
+        self.kps_lowres, self.K, self.kp_ld = subpixel_deconv_conv(torch, blobs); add(self.kps_lowres)
         self.loss_heads = torch.zeros(4, dtype=torch.float32, device='cuda')      # cls, bbox, kps, #correct
         self.totals = torch.zeros(2, dtype=torch.float32, device='cuda')          # live RoIs, keypoint weight sum (loss normalisers)
         self.iter = 0
@@ -567,18 +617,7 @@ class KeypointRcnnTrainer(RpnTrainer):
         for i, c in enumerate(self.kps):
             out['conv_fcn%d_w' % (i + 1)] = self._blob_w(c, blobs['conv_fcn%d_w' % (i + 1)].shape).astype(np.float32)
             out['conv_fcn%d_b' % (i + 1)] = c.bias.cpu().numpy()
-        K = self.K
-        w3 = self._blob_w(self.kps_lowres, (self.kp_ld, self.kps_lowres.cin, 3, 3))        # [ldk, cin, 3, 3]
-        wt = np.zeros_like(blobs['kps_score_lowres_w'])                                  # (cin, K, 4, 4)
-        for py in range(2):
-            for px in range(2):
-                for dy in (-1, 0, 1):
-                    for dx in (-1, 0, 1):
-                        ky, kx = py + 1 - 2 * dy, px + 1 - 2 * dx
-                        if 0 <= ky <= 3 and 0 <= kx <= 3:
-                            wt[:, :, ky, kx] = w3[(py * 2 + px) * K:(py * 2 + px + 1) * K, :, dy + 1, dx + 1].T
-        out['kps_score_lowres_w'] = wt
-        out['kps_score_lowres_b'] = self.kps_lowres.bias.cpu().numpy()[:K].copy()
+        export_subpixel_deconv(self, blobs, out)
         return out
 
     # ------------------------------------------------------------------ geometry / proposals

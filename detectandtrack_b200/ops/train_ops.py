@@ -153,6 +153,47 @@ def frcnn_loss_grad(out, labels, targets, inside, outside, C_, totals, scale_cls
     return grad
 
 
+def frcnn_tube_loss_grad(out, labels, targets, inside, outside, T, C_, totals, scale_cls, scale_box, ld_g, loss=None, accuracy=None):
+    """out [R*T, ld_o] fp32 per RoI-frame (C_ logits | 4C_ deltas) -> grad [R*T, ld_g] bf16 through the tube fold;
+    labels [R], targets / weights [R, 4*C_*T]; loss [2] += (cls, bbox)."""
+    torch = L.require_cuda()
+    rows, ld_o = out.shape
+    assert rows % T == 0
+    grad = torch.empty((rows, ld_g), dtype=torch.bfloat16, device='cuda')
+    L.call('dt_frcnn_tube_loss_grad', L.ptr(out), ld_o, L.ptr(labels), L.ptr(targets), L.ptr(inside), L.ptr(outside), rows // T, T, C_,
+           L.ptr(totals), float(scale_cls), float(scale_box), L.ptr(grad), ld_g, L.ptr(loss), L.ptr(accuracy), L.stream_ptr())
+    return grad
+
+
+def rpn_tube_loss_grad(out, A, t, scale_cls, scale_box, ld_g, loss=None, normalizer=None, beta=1.0 / 9.0):
+    """out [B, T, H, W, ld_o] fp32 per-frame RPN output; t: dt_rpn_targets dict (labels [B,H,W,A], bbox_targets / inside /
+    outside [B,H,W,4TA]) -> grad [B, T, H, W, ld_g] bf16; loss [2] += (cls, bbox).  normalizer: [1] fp32 scratch that
+    receives the SigmoidCrossEntropyLoss normaliser max(#labels >= 0, 1e-5)."""
+    torch = L.require_cuda()
+    B, T, H, W, ld_o = out.shape
+    assert out.dtype == torch.float32 and out.is_contiguous()
+    if normalizer is None:
+        normalizer = torch.empty((1,), dtype=torch.float32, device='cuda')
+    grad = torch.empty((B, T, H, W, ld_g), dtype=torch.bfloat16, device='cuda')
+    L.call('dt_rpn_tube_loss_grad', L.ptr(out), ld_o, L.ptr(t['labels']), L.ptr(t['bbox_targets']), L.ptr(t['inside']), L.ptr(t['outside']),
+           B, T, H, W, A, float(scale_cls), float(scale_box), float(beta), L.ptr(normalizer), L.ptr(grad), ld_g, L.ptr(loss), L.stream_ptr())
+    return grad
+
+
+def spatial_mean_bwd(g, hw, y=None, scale=None, second=False, scale2=None):
+    """g [N, C] bf16 (gradient wrt the spatial mean) -> [N, H, W, C] = g / (H*W) * [y > 0] * scale[c]; second=True also returns
+    the same masked value times scale2[c] (or unscaled), like bwd_pointwise(second=True)."""
+    torch = L.require_cuda()
+    N, Cc = g.shape
+    H, W = hw
+    assert g.dtype == torch.bfloat16 and g.is_contiguous()
+    assert y is None or (y.dtype == torch.bfloat16 and y.is_contiguous() and tuple(y.shape) == (N, H, W, Cc))
+    out = torch.empty((N, H, W, Cc), dtype=torch.bfloat16, device='cuda')
+    out2 = torch.empty_like(out) if second else None
+    L.call('dt_spatial_mean_bwd', L.ptr(g), N, H, W, Cc, L.ptr(y), L.ptr(scale), L.ptr(out), L.ptr(scale2), L.ptr(out2), L.stream_ptr())
+    return (out, out2) if second else out
+
+
 def kps_loss_grad(low, K, locations, weights, totals, scale, ld_g, loss=None):
     """low [D, S, S, ld] fp32 (sub-pixel packed kps_score_lowres) -> grad [D, S, S, ld_g] bf16 of the spatial-softmax loss."""
     torch = L.require_cuda()

@@ -6,8 +6,9 @@
 
 The loop: minibatch (TRAIN.IMS_PER_BATCH clips + their ground truth) -> trainer.step (forward, device-side targets, losses,
 backward, bucketed gradient all-reduce, SGD with the lr of lib/utils/lr_policy) -> smoothed loss log every 20 iterations.
-TRAIN.DATASET 'synthetic_VxF[_HxW]' draws seeded frames and persons; any other name is a JSON list of roidb entries with
-'image', 'height', 'width', 'boxes', 'gt_keypoints' (the fields lib/datasets/json_dataset.py builds).
+TRAIN.DATASET 'synthetic_VxF[_HxW]' draws seeded frames and persons (person tubes for the 3-D tube models); any other name is a
+JSON list of roidb entries with 'image', 'height', 'width', 'boxes', 'gt_keypoints' (the fields lib/datasets/json_dataset.py
+builds; [G,4T] boxes and [G,3,K*T] keypoints for tube models).
 """
 import argparse
 import logging
@@ -45,18 +46,34 @@ def find_resume_point(output_dir):
     return start, path
 
 
-def _synthetic_gt(entry, K):
+def _synthetic_gt(entry, K, T=1):
+    """Seeded persons of a synthetic clip.  T > 1: tubes, boxes [G,4T] with every frame's box the T == 1 draw shifted by up to
+    3 % of the frame size (clipped to the frame), keypoints [G,3,K*T] drawn per frame inside that frame's box."""
     rng = np.random.RandomState(entry['seed'] % (2 ** 31))
     H, W, G = entry['height'], entry['width'], 3
     w = rng.uniform(0.08, 0.2, G) * W; h = rng.uniform(0.2, 0.4, G) * H
     x1 = rng.uniform(0, W - 1 - w); y1 = rng.uniform(0, H - 1 - h)
     boxes = np.stack([x1, y1, x1 + w, y1 + h], 1).astype(np.float32)
-    kps = np.zeros((G, 3, K), np.int32)
+    if T == 1:
+        kps = np.zeros((G, 3, K), np.int32)
+        for i in range(G):
+            kps[i, 0] = rng.randint(int(boxes[i, 0]), int(boxes[i, 2]) + 1, K)
+            kps[i, 1] = rng.randint(int(boxes[i, 1]), int(boxes[i, 3]) + 1, K)
+            kps[i, 2] = rng.randint(0, 3, K)
+        return dict(boxes=boxes, gt_keypoints=kps)
+    shift = rng.uniform(-0.03, 0.03, (G, T, 2)) * np.array([W, H])
+    tubes = np.zeros((G, T, 4), np.float32)
+    for t in range(T):
+        b = boxes + np.tile(shift[:, t], 2)
+        tubes[:, t] = np.clip(b, 0, [W - 1, H - 1, W - 1, H - 1])
+    kps = np.zeros((G, 3, K * T), np.int32)
     for i in range(G):
-        kps[i, 0] = rng.randint(int(boxes[i, 0]), int(boxes[i, 2]) + 1, K)
-        kps[i, 1] = rng.randint(int(boxes[i, 1]), int(boxes[i, 3]) + 1, K)
-        kps[i, 2] = rng.randint(0, 3, K)
-    return dict(boxes=boxes, gt_keypoints=kps)
+        for t in range(T):
+            bx = tubes[i, t]
+            kps[i, 0, t * K:(t + 1) * K] = rng.randint(int(bx[0]), int(bx[2]) + 1, K)
+            kps[i, 1, t * K:(t + 1) * K] = rng.randint(int(bx[1]), int(bx[3]) + 1, K)
+            kps[i, 2, t * K:(t + 1) * K] = rng.randint(0, 3, K)
+    return dict(boxes=tubes.reshape(G, 4 * T), gt_keypoints=kps)
 
 
 def train_model():
@@ -92,6 +109,7 @@ def train_model():
         log.info('Wrote %s', path)
     roidb = te.get_dataset(cfg.TRAIN.DATASET).get_roidb(gt=True)
     K = cfg.KRCNN.NUM_KEYPOINTS
+    T = P.GraphSpec(cfg).T_head                    # frames per gt tube (1: boxes)
     B = cfg.TRAIN.IMS_PER_BATCH
     order = np.random.RandomState(cfg.RNG_SEED).permutation(len(roidb))
     smooth = []
@@ -99,7 +117,7 @@ def train_model():
         idx = [order[(it * world * B + rank * B + j) % len(order)] for j in range(B)]
         entries = [roidb[i] for i in idx]
         frames = torch.from_numpy(np.stack([np.stack(te.read_image_video(e)) for e in entries])).cuda()
-        gts = [(_synthetic_gt(e, K) if e.get('synthetic') else dict(boxes=np.asarray(e['boxes'], np.float32),
+        gts = [(_synthetic_gt(e, K, T) if e.get('synthetic') else dict(boxes=np.asarray(e['boxes'], np.float32),
                                                                     gt_keypoints=np.asarray(e['gt_keypoints'], np.int32))) for e in entries]
         model.lr = float(get_lr_at_iter(it))
         l_rpn, l_heads = model.step(frames, pack_gt(gts, K=K))
