@@ -14,7 +14,8 @@
 //   n = output channel, BLOCK_N in {32, 64, 128, 256};  k-block = one tap x 128 bytes of channels
 //   A tile: one 5-D TMA box (C=128B, TW, TH, 1, 1) at the tap-shifted coordinate; out-of-bounds
 //           elements (spatial / temporal zero padding, ragged edge tiles, channel tail) are
-//           zero-filled by the TMA unit, so padding costs no instructions and no branches.
+//           zero-filled by the TMA unit, so padding costs no instructions and no branches.  Taps of the outermost
+//           filter dimension whose box lies wholly in that fill are not issued at all (tap_range).
 //   W tile: 3-D TMA box (C=128B, BLOCK_N, 1) of the pre-packed [tap][Cout][Cin] weights.
 //   Both land in the 128B-swizzled K-major layout tcgen05.mma reads directly.
 // Roles (640 threads, 1 CTA / SM, persistent over tiles):
@@ -82,6 +83,8 @@ struct ConvKernelParams {
   int ks;                      // k-blocks per ring stage
   int ktab;                    // entries of the k-block schedule (kiters + 1 padding, even)
   int t_first;                 // first output frame computed (frames before it are skipped)
+  int Ti, Hi;                  // input frames / rows (the extents tap_range tests a tap's box against)
+  int tap_skip;                // 1: each tile walks only the taps of tap_range (0: every tap)
   int row_planes;              // conv1: input rows de-interleaved by parity, filter row kh -> plane kh & 1, row + kh >> 1
   int nrbuf;                   // > 0: bf16 residual chunks arrive by TMA in a ring of this many staged chunks
   int res_up;                  // with nrbuf > 0: the residual is the (Ho/2, Wo/2) map of the FPN top-down add;
@@ -144,6 +147,33 @@ __device__ __forceinline__ TileCoord decode_tile(const ConvKernelParams& p, int 
   q = fdiv(m, p.fd_t);                        c.tti = (int)m - (int)q * p.tiles_t;
   c.tbi = (int)q;
   return c;
+}
+
+// Schedule entries [kb, ke) one tile issues.  The schedule is tap-major with kt outermost, so the taps of the
+// outermost filter dimension with more than one tap (kt, else kh) are contiguous runs of kiters / extent entries.
+// Tap k of that dimension reads input positions base + k + j*s, j in [0, n) (n = TT frames or TH rows of the tile's
+// box); when none of them lies inside [0, lim) the box is all TMA zero fill and its products are exact zeros, so
+// those taps are left out.  Skipping zero products and keeping the order of the others leaves every sum unchanged.
+// An empty range (a tile wholly in the padding) issues everything, so the accumulator is always written.
+struct KRange { int kb, ke; };
+__device__ __forceinline__ KRange tap_range(const ConvKernelParams& p, const TileCoord& tc, int kiters) {
+  KRange r = {0, kiters};
+  if (!p.tap_skip) return r;
+  int ext, base, n, s, lim;
+  if (p.kT > 1) {
+    ext = p.kT; base = (tc.tti * p.TT + p.t_first) * p.sT - p.pT; n = p.TT; s = p.sT; lim = p.Ti;
+  } else if (p.kH > 1) {
+    ext = p.kH; base = tc.thi * p.TH * p.sH - p.pH; n = p.TH; s = p.sH; lim = p.Hi;
+  } else {
+    return r;
+  }
+  const int k0 = max(0, -(base + (n - 1) * s));
+  const int k1 = min(ext, lim - base);
+  if (k0 < k1) {
+    const int per = kiters / ext;
+    r.kb = k0 * per; r.ke = k1 * per;
+  }
+  return r;
 }
 
 #ifdef DT_CONV_TRACE
@@ -266,12 +296,13 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       const int h_base = tc.thi * p.TH * p.sH - p.pH;
       const int t_base = p.row_planes ? 0 : (tc.tti * p.TT + p.t_first) * p.sT - p.pT;
       const int n_base = tc.nt * BN;
+      const KRange kr = tap_range(p, tc, kiters);
 #ifdef DT_CONV_TRACE
       long long acc_wait = 0, acc_issue = 0;
 #endif
       if (lane == 0 && !load_b) TRACE(tile / gridDim.x, 0);
-      for (int ki = 0; ki < kiters; ki += KS) {
-        const int nk = min(KS, kiters - ki);
+      for (int ki = kr.kb; ki < kr.ke; ki += KS) {
+        const int nk = min(KS, kr.ke - ki);
         // this stage's k-blocks from the schedule (uniform loads), then ONE elected issue block
         int x0[2], x1[2], x2[2], x3[2];
 #pragma unroll
@@ -346,12 +377,13 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       mbar_wait(&tmem_empty[as], aphase ^ 1);
       tcgen05_fence_after();
       const uint32_t d_tmem = tmem_u + as * BN;
+      const KRange kr = tap_range(p, decode_tile(p, tile), kiters);     // the producers' range: the rings stay in step
       if (lane == 0) TRACE(tile / gridDim.x, 2);
 #ifdef DT_CONV_TRACE
       long long acc_wf = 0;
 #endif
-      for (int ki = 0; ki < kiters; ki += KS) {
-        const int nk = min(KS, kiters - ki);
+      for (int ki = kr.kb; ki < kr.ke; ki += KS) {
+        const int nk = min(KS, kr.ke - ki);
 #ifdef DT_CONV_TRACE
         const long long tw1 = clock64();
 #endif
@@ -367,10 +399,10 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             const uint64_t bdesc = make_sw128_kmajor_desc(a_addr + q * Cfg::KB_BYTES + Cfg::A_BYTES);
 #pragma unroll
             for (int k = 0; k < 4; ++k)          // 4 x 32 B = one 128-byte swizzle row of K
-              umma<TF32>(d_tmem, adesc + 2 * k, bdesc + 2 * k, idesc, (ki | q | k) != 0 ? 1u : 0u);
+              umma<TF32>(d_tmem, adesc + 2 * k, bdesc + 2 * k, idesc, (ki != kr.kb || q || k) ? 1u : 0u);
           }
           umma_commit(&empty[stage]);            // frees the smem slot when these MMAs retire
-          if (ki + nk >= kiters) umma_commit(&tmem_full[as]);   // accumulator ready for the epilogue
+          if (ki + nk >= kr.ke) umma_commit(&tmem_full[as]);   // accumulator ready for the epilogue
         }
         if (++stage == STAGES) { stage = 0; phase ^= 1; }
       }
@@ -827,6 +859,13 @@ extern "C" int dt_conv3d(const dt_conv_desc* d, const void* x, const void* w, co
                        ((uintptr_t)residual % 16) == 0;
   if (res_tma && BN > 128) BN = 128;
   p.t_first = d->out_t_count > 0 ? d->out_t_first : 0;
+  p.Ti = d->Ti; p.Hi = d->Hi;
+  // DT_CONV_TAP_SKIP=0 in the environment issues every tap of every tile (the same results, for A/B timing); read on
+  // each call, unlike DT_PDL, so that one process can run a conv both ways
+  {
+    const char* e = getenv("DT_CONV_TAP_SKIP");
+    p.tap_skip = (e && e[0] == '0') ? 0 : 1;
+  }
   p.nrbuf = res_tma ? 1 : 0;                         // ring depth is chosen with the smem split at launch
   p.res_up = (res_tma && d->res_mode == 2) ? 1 : 0;
   p.tiles_n = cdiv(d->Cout, BN);
